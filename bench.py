@@ -2,6 +2,14 @@
 """bench.py -- rays/sec of the SDF volume-rendering hot path (BASELINE.json metric), one workload per invocation.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--precision bf16x3|bf16|fp32]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the timed path returned in its last timed step as DIR/<name>.npy
+          (float32; at most 64 MB in all).  Inputs and parameters are seeded, so two builds run with the same arguments can be compared
+          output for output.  Render workloads: the arrays SDFField.render returns (rgb, depth, normal, accumulation, bg_transmittance,
+          weights).  angelo-train-8192: the loss and a fixed, seeded sample of every parameter after the optimizer step.  k_field_tc adds
+          the per-warp partial sums of a ray in shared memory with atomics (S > 32), so the rendered values of two runs may differ in
+          the last bits: compare with a tolerance.
 
 Workloads (BASELINE.json configs; the default is the headline the metric is quoted on):
   neus-facto-dtu65-4096x128   configs[1]: DTU-scan65-shaped rays, 4096 rays x 128 samples per GPU, neus-facto SDFField (hash L=16 F=2
@@ -45,6 +53,20 @@ WORKLOAD = "neus-facto-dtu65-4096x128"
 WORKLOADS = (WORKLOAD, "volsdf-errorbounded-4096", "bakedsdf-render-65536", "angelo-train-8192")
 AABB = [[-1.0, -1, -1], [1, 1, 1]]
 VOLSDF_BETA = 0.01   # Laplace beta of the volsdf workload: small like a trained scene, so that the error-bounded refinement loop actually iterates
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor} as out_dir/<name>.npy in float32 (float64 stays float64)."""
+    import numpy as np
+
+    arrs = {k: v.detach().cpu().to(torch.float64 if v.dtype == torch.float64 else torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrs.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES} byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------------ fields
@@ -246,7 +268,7 @@ def run_reference(args):
     full = args.workload == WORKLOAD
     rays = R_PER_GPU if full else 256
     warm = max(min(args.warmup, 3), 1) if not full else 1
-    steps = max(1, min(args.steps, 10 if full else 20))
+    steps = args.steps
     value, dt, cores = cpu_arm(args.workload, rays, steps, warm)
     sample = f"{rays} rays per step ({'the full batch' if full else 'bounded sample'}) of the {args.workload} step ({dt * 1e3:.0f} ms/step), {steps} steps after {warm} warm-up"
     line = {
@@ -302,7 +324,12 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="A/B: e2e without CUDA-graph replay")
     ap.add_argument("--no-train-section", action="store_true", help="skip the training-step section (angelo-train-8192 with the NCCL gradient all-reduce) of the headline line")
     ap.add_argument("--table-dtype", default="fp32", choices=["fp32", "fp16"], help="fp16 = gather from a half-precision copy (tiny-cuda-nn's storage)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "angelo-train-8192":
@@ -532,7 +559,7 @@ def main():
     train = None
     if wl == WORKLOAD and not args.no_train_section:
         torch.cuda.empty_cache()
-        train = train_section(world, rank)
+        train = train_section(world, rank, args.steps, args.warmup)
         barrier()
     times = torch.tensor([dev_ms, e2e_ms, fld_ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -566,6 +593,8 @@ def main():
         line.update(extra)
         if train is not None:
             line["training_step"] = train
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {k: v for k, v in last.items() if isinstance(v, torch.Tensor)})
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -9,20 +9,16 @@ if ROOT not in sys.path:
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "gpu: needs a CUDA device (select with -m gpu)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir("/root/reference/nerfstudio")
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present"))
 
 
 @pytest.fixture(scope="session")

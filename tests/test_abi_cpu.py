@@ -228,23 +228,38 @@ def test_proposal_network_checkpoint_layout_loads():
         checkpoint.load_density_field_checkpoint(wrong, ckpt, index=0)
 
 
-@pytest.mark.reference
+def _reference_tensordataclasses():
+    """(RayBundle class, RaySamples of the reference's UniformSampler, FieldHeadNames values) rebuilt from the fixture minted from the
+    unmodified reference by oracle/make_golden_tensordataclass.py: classes with the reference's dataclass fields, and every tensor of the
+    RaySamples with the reference's exact shape, stride, storage offset and storage sharing."""
+    import dataclasses
+    import json
+
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_tensordataclass.json")) as fh:
+        fx = json.load(fh)
+    cls = {name: dataclasses.make_dataclass(name, [(f, object) if required else (f, object, dataclasses.field(default=None)) for f, required in fx[name]])
+           for name in ("RayBundle", "RaySamples", "Frustums")}
+    storages = [torch.tensor(s["data"], dtype=getattr(torch, s["dtype"])) for s in fx["storages"]]
+    views = {name: storages[v["storage"]].as_strided(v["shape"], v["stride"], v["offset"]) for name, v in fx["ray_samples"].items()}
+    frustums = cls["Frustums"](**{k.split(".", 1)[1]: v for k, v in views.items() if k.startswith("frustums.")})
+    rs = cls["RaySamples"](frustums=frustums, **{k: v for k, v in views.items() if not k.startswith("frustums.")})
+    for name, v in fx["ray_samples"].items():
+        t = views[name]
+        assert list(t.shape) == v["shape"] and list(t.stride()) == v["stride"] and t.storage_offset() == v["offset"], name
+    return cls["RayBundle"], rs, fx["FieldHeadNames"]
+
+
 def test_reference_tensordataclasses_pass_through_the_host_side():
     """The reference's own RayBundle / RaySamples (TensorDataclass objects with expanded stride-0 fields, cameras/rays.py:233-339) are what the
     modules receive inside sdfstudio: the host-side accessors must read them, keep their TYPE when slicing / flattening, and rebuild the
-    [R, S+1] bin buffer the kernels take.  Structure only (no kernel runs on the CPU box)."""
-    from oracle import ref_import
+    [R, S+1] bin buffer the kernels take.  Structure only: no kernel runs."""
+    from oracle.make_golden_tensordataclass import H, W, S, camera_bundle_inputs
 
     import sdfstudio_b200 as sb
     from sdfstudio_b200 import parallel
 
-    ref = ref_import.ref_modules()
-    H, W, S = 5, 7, 9
-    g = torch.Generator().manual_seed(2)
-    d = torch.randn(H, W, 3, generator=g)
-    d = d / d.norm(dim=-1, keepdim=True)
-    bundle = ref.RayBundle(origins=torch.randn(H, W, 3, generator=g), directions=d, pixel_area=torch.ones(H, W, 1), directions_norm=torch.ones(H, W, 1),
-                           camera_indices=torch.zeros(H, W, 1, dtype=torch.long), nears=torch.full((H, W, 1), 0.5), fars=torch.full((H, W, 1), 4.5))
+    RayBundle, rs, ref_heads = _reference_tensordataclasses()
+    bundle = RayBundle(**camera_bundle_inputs())
     flat, hw = parallel.flatten_ray_bundle(bundle)
     assert hw == (H, W) and type(flat) is type(bundle) and flat.origins.shape == (H * W, 3) and flat.camera_indices.dtype == torch.long
     assert torch.equal(flat.origins.view(H, W, 3), bundle.origins)
@@ -252,9 +267,8 @@ def test_reference_tensordataclasses_pass_through_the_host_side():
     assert type(part) is type(bundle) and part.origins.shape == (8, 3) and torch.equal(part.fars, flat.fars[3:11])
     sh = parallel.shard_ray_bundle(flat, 1, 3)
     assert sh.origins.shape[0] == parallel.shard_bounds(H * W, 1, 3)[1] - parallel.shard_bounds(H * W, 1, 3)[0]
-    # the reference sampler's RaySamples: starts / ends are overlapping slices of one bin buffer, origins / directions stride-0 expanded
-    rs = ref.ray_samplers.UniformSampler(num_samples=S).eval()(flat)
-    assert rs.frustums.origins.stride()[1] == 0
+    # the reference sampler's RaySamples of `flat`: starts / ends are overlapping slices of one bin buffer, origins / directions stride-0 expanded
+    assert rs.frustums.origins.stride()[1] == 0 and rs.frustums.starts.untyped_storage().data_ptr() == rs.frustums.ends.untyped_storage().data_ptr()
     bins = sb.rays.bins_of(rs)
     assert bins.shape == (H * W, S + 1) and bins.is_contiguous()
     assert torch.equal(bins[:, :-1], rs.frustums.starts[..., 0]) and torch.equal(bins[:, 1:], rs.frustums.ends[..., 0])
@@ -263,8 +277,7 @@ def test_reference_tensordataclasses_pass_through_the_host_side():
     o2, d2 = sb.rays.rays_of(rs)
     assert o2.is_contiguous() and torch.equal(o2, flat.origins) and torch.equal(d2, flat.directions)
     # FieldHeadNames of the reference compare equal to the product's keys (dicts returned by SDFField are indexed with either)
-    assert {h.value for h in ref.FieldHeadNames} >= {h.value for h in sb.FieldHeadNames} or all(
-        getattr(ref.FieldHeadNames, h.name).value == h.value for h in sb.FieldHeadNames)
+    assert set(ref_heads.values()) >= {h.value for h in sb.FieldHeadNames} or all(ref_heads[h.name] == h.value for h in sb.FieldHeadNames)
 
 
 def test_grouped_grid_calls_reject_bad_groups_and_encoding_context_nests():

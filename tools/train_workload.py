@@ -133,6 +133,14 @@ def main(args):
     barrier()
     launches = sb._lib.launch_count() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in pairs)
+    if args.dump_outputs and rank == 0:
+        # the loss and a fixed, seeded sample (<= 65536 entries) of every parameter as the last timed step left them
+        g_dump = torch.Generator().manual_seed(0)
+        dumped = {"loss": loss.clone()}
+        for name, p in field.named_parameters():
+            flat = p.detach().reshape(-1)
+            idx = torch.randint(0, flat.numel(), (65536,), generator=g_dump).sort().values if flat.numel() > 65536 else torch.arange(flat.numel())
+            dumped["param." + name] = flat[idx.to(dev)].clone()
     # end to end: host rays in, scalar loss out (the reference's train_iteration returns the loss dict to the host: trainer.py:319-327)
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
     pairs2 = []
@@ -191,6 +199,8 @@ def main(args):
                          "algorithmic_bytes_per_step": table_bytes},
             "cpu_baseline": None, "clocks": clk, "loss": float(loss),
         }
+        if args.dump_outputs:
+            bench.dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -204,4 +214,5 @@ if __name__ == "__main__":
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--precision", default="auto")
+    ap.add_argument("--dump-outputs", metavar="DIR")
     main(ap.parse_args())
